@@ -144,6 +144,13 @@ class CpuReference:
         return n_faces / dt, dt
 
 
+def dump_outputs(out_dir, named):
+    """Write each output tensor as out_dir/<name>.npy in float32, so that two builds can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in named.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
 def workload_config(B):
     return {"workload": WORKLOAD, "batch_per_gpu": B, "input": "uint8 256x256x3 crops",
             "l2": "inputs rotate over 4 x 50 MB sets (> 126 MB L2); activations per batch exceed L2"}
@@ -190,7 +197,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-pipeline", action="store_true", help="skip the full-pipeline (configs 3/5) and detector legs")
     ap.add_argument("--pipeline-streams", type=int, default=16)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the landmarks and scores of the last timed step (rank 0) as DIR/<name>.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -273,6 +286,10 @@ def main():
         ms = float(t.item())
     faces_per_s = whole_job_rate(world, B, args.steps, ms * 1e-3)
     log("device-resident: %.1f faces/s (%.3f ms/step)" % (faces_per_s, ms / args.steps))
+    if args.dump_outputs and rank == 0:
+        # `outs` is written by the timed steps only: it holds the last step's results (input set (steps - 1) % n_sets)
+        dump_outputs(args.dump_outputs, {"landmarks": outs[0], "scores": outs[1]})
+        log("outputs of the last timed step written to %s" % args.dump_outputs)
 
     # ---- end to end through the operator call with host buffers (pinned), H2D + D2H inside the timed region
     e2e_steps = max(5, min(args.steps, 20))

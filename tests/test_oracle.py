@@ -13,6 +13,31 @@ def sha(a):
     return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
 
 
+# The fixtures were recorded with the oracle's torch-CPU executor on one host.  Its float32 convolutions round differently with
+# the CPU's vector width and thread count (a few float32 ulps; its float32 vs float64 gap on the detector is 1e-4 / 7e-7 relative),
+# so executor outputs are compared within these bounds, while the host code, fed the recorded network outputs, must match exactly.
+DET_ROW_RTOL = 1e-5                  # detector rows: |d| <= DET_ROW_RTOL * (1 + |v|)
+KPS_NET_TOL_PX, KPS_NET_TOL_SCORE = 2e-4, 2e-5      # twice test_student_executor_fp64_tie_breaker's float32 vs float64 bound
+RUN_TOL_PX, RUN_TOL_SCORE = 5e-4, 2e-5              # whole run(): landmarks and boxes in frame pixels
+
+
+class _Replay:
+    """Stands in for an oracle executor Session: returns recorded network outputs in call order."""
+
+    def __init__(self, outputs):
+        self.outputs = list(outputs)
+
+    def run(self, x):
+        return self.outputs.pop(0)
+
+
+def _recorded_det_raw(g, t):
+    """The detector output of frame t as far as the fixture keeps it: every row scoring over 0.25 (NMS reads rows over 0.5)."""
+    raw = np.zeros((15120, 16), np.float32)
+    raw[g["f%d_det_cand_idx" % t]] = g["f%d_det_cand_rows" % t]
+    return raw
+
+
 @pytest.mark.parametrize("shape,dst", [
     ((273, 410), (640, 426)), ((1080, 1920), (640, 360)), ((2160, 3840), (640, 360)),
     ((214, 214), (256, 256)), ((97, 97), (256, 256)), ((300, 301), (256, 256)),
@@ -49,8 +74,13 @@ def test_detector_restated_matches_golden(golden, ref_nets):
         g = golden(name)
         raw, recover, _ = det.raw(fr)
         raw = np.asarray(raw).reshape(15120, 16)
-        assert sha(raw) == str(g["f0_det_raw_sha"])
+        cand = g["f0_det_cand_idx"]
+        assert np.array_equal(np.where(raw[:, 4] > 0.25)[0], cand)
+        ref = g["f0_det_cand_rows"]
+        assert (np.abs(raw[cand] - ref) <= DET_ROW_RTOL * (1 + np.abs(ref))).all(), np.abs(raw[cand] - ref).max()
         kept, idx = H.detect_post(raw, recover)
+        assert np.array_equal(idx, g["f0_det_keep_idx"])
+        kept, idx = H.detect_post(_recorded_det_raw(g, 0), recover)
         assert np.array_equal(idx, g["f0_det_keep_idx"])
 
 
@@ -65,8 +95,8 @@ def test_crop_and_landmarks_match_golden(golden, ref_nets):
             assert np.array_equal(crop, g["f0_crops"][i])
             assert list(detail) == list(g["f0_details"][i])
         xy, sc = kps.forward_crops(g["f0_crops"][:2])
-        assert np.array_equal(xy.reshape(len(xy), -1), g["f0_kps_raw"][:2])
-        assert np.array_equal(sc, g["f0_kps_score"][:2])
+        assert np.abs(xy.reshape(len(xy), -1) - g["f0_kps_raw"][:2]).max() * 256 <= KPS_NET_TOL_PX
+        assert np.abs(sc - g["f0_kps_score"][:2]).max() <= KPS_NET_TOL_SCORE
 
 
 def test_heatmap_decode_matches_graph(ref_nets, golden):
@@ -86,10 +116,20 @@ def test_faceana_restated_matches_reference_video(golden):
     from oracle.faceana_ref import FaceAnaRef
     from golden.make_golden_frames import video_frames
     g = golden("video1080")
-    f = FaceAnaRef()
+    live, replay = FaceAnaRef(), FaceAnaRef()
     for t, fr in enumerate(video_frames()):
-        res = f.run(fr.copy())
-        assert len(res) == int(g["f%d_res_n" % t])
+        n = int(g["f%d_res_n" % t])
+        res = live.run(fr.copy())
+        assert len(res) == n
+        if res:
+            assert np.abs(np.stack([r["kps"] for r in res]) - g["f%d_res_kps" % t]).max() <= RUN_TOL_PX
+            assert np.abs(np.stack([r["scores"] for r in res]) - g["f%d_res_scores" % t]).max() <= RUN_TOL_SCORE
+            assert np.abs(np.stack([r["box"] for r in res]) - g["f%d_res_box" % t]).max() <= RUN_TOL_PX
+        # the same frame through the host code with the networks replaced by the outputs recorded from the reference
+        replay.det.net = _Replay([[_recorded_det_raw(g, t)]] if "f%d_det_cand_idx" % t in g else [])
+        replay.kps.net = _Replay(zip(g["f%d_kps_raw" % t], g["f%d_kps_score" % t]) if "f%d_kps_raw" % t in g else [])
+        res = replay.run(fr.copy())
+        assert len(res) == n and not replay.det.net.outputs and not replay.kps.net.outputs
         if res:
             assert np.array_equal(np.stack([r["kps"] for r in res]).astype(np.float32), g["f%d_res_kps" % t])
             assert np.array_equal(np.stack([r["scores"] for r in res]), g["f%d_res_scores" % t])
